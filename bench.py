@@ -10,10 +10,14 @@ roofline), `imagination_update` (cfg 3: 32 envs x horizon 15 through WorldModelE
 `gpu_baseline` (the reference's GPU path on this GPU: eager and torch.compile), `cpu_baseline` (its CPU path on the host cores).
 Multi-GPU is weak scaling: imagination needs no collective (SURVEY.md 8e); both training blocks all-reduce their gradients.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--envs B] [--impl native|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--envs B] [--impl native|reference] [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  `--impl reference` times the reference algorithm's CPU path (the oracle port — the
 reference is pure Python and /root/reference does not travel to the GPU box) on the host cores.
+
+`--dump-outputs DIR` also writes what the last timed sample() call returned (rank 0's environments) as DIR/x.npy and
+DIR/trajectory.npy.  Inputs and sampler noise are seeded, so two builds run with the same arguments can be compared output
+for output.
 """
 import argparse
 import json
@@ -26,10 +30,12 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 METRIC = "imagined frames/sec (64x64, 3 denoise steps)"
 GFLOP_PER_FRAME = 18.266  # SURVEY.md 8d: 3 x 6.0888 GFLOP denoiser forwards
 TRS = os.environ.get("DMD_CONV_TRS", "0") != "0"  # the executor's weight layout for 3x3 convs (tap-major; DMD_CONV_TRS=1 selects the tap-row-stacked experiment)
+DUMP_LIMIT_BYTES = 64 << 20
 
 
 def load_peaks():
@@ -145,7 +151,7 @@ def run_reference(args):
     torch.set_num_threads(cores)
     cfg, sc = O.DenoiserCfg(inner=inner), O.SamplerCfg(3)
     obs, act, x0 = O.synthetic_inputs(envs, inner, 64, 64, 5)
-    steps = min(args.steps, 8)  # bounded: K x 32 envs x 3 U-Net forwards on the host cores
+    steps = args.steps
     warmups = 0
     with torch.no_grad():
         for _ in range(max(1, min(args.warmup, 2))):
@@ -153,15 +159,16 @@ def run_reference(args):
             O.sample(obs, act, x0, sd, cfg, sc)
             t_one = time.perf_counter() - t0
             warmups += 1
-            if t_one > 15.0:      # a host shared with other jobs: keep the whole arm within ~2 minutes
+            if t_one > 15.0:      # a host shared with other jobs: at most one warm-up of a slow arm
                 break
-        steps = max(1, min(steps, int(90.0 / max(t_one, 1e-3))))
         t0 = time.perf_counter()
         for _ in range(steps):
-            O.sample(obs, act, x0, sd, cfg, sc)
+            x, traj = O.sample(obs, act, x0, sd, cfg, sc)
         dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, x, torch.stack(traj))
     val = envs * steps / dt
-    sample = f"{envs} envs x {steps} sample() calls (the full {args.envs}-env workload per step; steps capped at 8 and at ~90 s of work), torch {torch.__version__} CPU fp32, {cores} threads (fastest of 8/16/32/64/{avail} available)"
+    sample = f"{envs} envs x {steps} sample() calls (the full {args.envs}-env workload per step), torch {torch.__version__} CPU fp32, {cores} threads (fastest of 8/16/32/64/{avail} available)"
     print(json.dumps({
         "impl": "reference", "metric": METRIC, "value": val, "unit": "frames/s", "n_gpus": args.gpus, "steps": steps,
         "warmup": warmups, "ms_per_step": 1e3 * dt / steps, "higher_is_better": True, "scaling": "weak",
@@ -170,6 +177,23 @@ def run_reference(args):
         "cpu_baseline": {"value": val, "unit": "frames/s", "cores": cores, "kind": "port", "sample": sample},
         "e2e": {"value": val, "unit": "frames/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }))
+
+
+def dump_outputs(out_dir: str, x, traj) -> None:
+    """What one sample() call returned -- the next frames x (B, C, H, W) and the denoising trajectory (num_sigmas, B, C, H, W)
+    -- as float32 out_dir/x.npy and out_dir/trajectory.npy.  When the two exceed DUMP_LIMIT_BYTES, a fixed seeded subset of
+    the B environments is written (the same rows of both, in ascending order)."""
+    import numpy as np
+    import torch
+
+    b = x.shape[0]
+    per_env = 4 * (x[0].numel() + traj[:, 0].numel())
+    keep = min(b, DUMP_LIMIT_BYTES // per_env)
+    rows = np.arange(b) if keep == b else np.sort(np.random.default_rng(0).choice(b, keep, replace=False))
+    rows = torch.from_numpy(rows).to(x.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "x.npy"), x.index_select(0, rows).float().cpu().numpy())
+    np.save(os.path.join(out_dir, "trajectory.npy"), traj.index_select(1, rows).float().cpu().numpy())
 
 
 def workload_config(args, envs_override=None):
@@ -581,6 +605,7 @@ def run_native(args):
     obs_d, act_d = obs.to(dev), act.to(dev)
     obs_h, act_h = obs.pin_memory(), act.pin_memory()
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
+    torch.manual_seed(0)  # sample() draws its initial noise from torch's generator: same arguments, same outputs
 
     def barrier():
         if world > 1:
@@ -599,12 +624,14 @@ def run_native(args):
         flush.zero_()
         a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         a.record()
-        sampler.sample(obs_d, act_d)
+        x, traj = sampler.sample(obs_d, act_d)
         b.record()
         evs.append((a, b))
     barrier()
     t_wall = time.perf_counter() - t_wall0
     launches = int(lib.dmd_launch_count(0))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, x, torch.stack(traj))
     dev_ms = sum(a.elapsed_time(b) for a, b in evs)
 
     # ---- end to end through the public API with host buffers (H2D of the frame stack + actions, D2H of the frame)
@@ -699,6 +726,8 @@ def main():
     ap.add_argument("--skip-train", action="store_true", help="omit the denoiser-training block (cfg 2)")
     ap.add_argument("--train-batch", type=int, default=256, help="denoiser training batch per GPU (config/trainer.yaml: 32; BASELINE cfg 2: 256)")
     ap.add_argument("--skip-gpu-baseline", action="store_true", help="omit the reference-GPU-path leg (eager + torch.compile of the oracle port)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed sample() call returned (rank 0) as DIR/x.npy and "
+                    "DIR/trajectory.npy, float32, at most 64 MB (a fixed seeded subset of the environments beyond that)")
     ap.add_argument("--secondary-budget", type=float, default=200.0, help="seconds shared by the blocks that follow the headline numbers (training, imagination, baselines); ~55 s are used on a healthy box")
     args = ap.parse_args()
     if args.impl == "reference":

@@ -1,6 +1,6 @@
 """Imagined-rollout driver for the actor-critic update: drop-in for the generator the reference builds with
 `make_env_loop` (src/coroutines/env_loop.py:12-74) — same `.send(num_steps)` protocol, same 9-tuple, same results bit for
-bit (tests/test_env_host_logic.py checks it against the live reference), different mechanics:
+bit (tests/test_env_host_logic.py checks it against the reference's recorded outputs), different mechanics:
 
 * results are written into tensors preallocated for the whole rollout instead of per-step lists that are stacked;
 * the bootstrap values are assembled once at the end with a single `where` over (dead, V(final obs), V(next obs)) instead of

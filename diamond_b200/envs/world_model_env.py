@@ -1,7 +1,7 @@
 """WorldModelEnv: the batched imagined environment of the actor-critic phase (reference surface:
 src/envs/world_model_env.py:25-139 — same constructor, `reset` / `step` / `predict_next_obs` / `predict_rew_end`, same
-results given the same RNG streams; tests/test_env_host_logic.py checks the index work bit for bit against the live
-reference).  The mechanics are B200-first:
+results given the same RNG streams; tests/test_env_host_logic.py checks the index work bit for bit against the reference's
+recorded outputs).  The mechanics are B200-first:
 
 * the frame stack and the action stack are DEVICE-RESIDENT RINGS (`_frames` (T, B, C, H, W), `_acts` (T, B)); the
   reference's two `roll` copies per step (world_model_env.py:74-75) are an index increment, and the native sampler reads the

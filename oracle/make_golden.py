@@ -280,8 +280,93 @@ def make_rew_end():
     print("rew_end_default logits rms", float(np.sqrt((out["burn_rew"] ** 2).mean())), "size", os.path.getsize(path))
 
 
+def _test_module(name):
+    """tests/<name>.py, loaded by path (tests/ is not a package): the fixtures below run the same helpers as the test."""
+    import importlib.util
+
+    spec = importlib.util.spec_from_file_location(name, os.path.join(ROOT, "tests", name + ".py"))
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    return mod
+
+
+def make_oracle_vs_reference():
+    """tests/test_oracle_vs_reference.py: the reference's denoise / model output on the small net of that test, and the EDM
+    pieces of its training forward (noise-level draw, apply_noise, conditioners, wrap) on one RNG stream."""
+    T = _test_module("test_oracle_vs_reference")
+
+    ns = ref_import.load()
+    D = ns.diffusion
+    torch.set_num_threads(8)
+    sd = O.seeded_state_dict(O.inner_model_shapes(T.INNER), T.WSEED)
+    den = build_reference(ns, T.INNER, sd)
+    obs, act, x = O.synthetic_inputs(3, T.INNER, 32, 32, T.ISEED)
+    sig = torch.tensor(T.SIGMAS)
+    obs_flat = obs.reshape(3, 12, 32, 32)
+    with torch.no_grad():
+        dn = den.denoise(x, sig, obs_flat, act)
+        mo = den.compute_model_output(x, obs_flat, act, den.compute_conditioners(sig))
+    edm = D.Denoiser(D.DenoiserConfig(D.InnerModelConfig(*T.EDM_INNER), 0.5, 0.3))
+    edm.setup_training(D.SigmaDistributionConfig(*T.EDM_SIGMA_DIST))
+    edm_x = torch.from_numpy(np.random.default_rng(94).random((5, 3, 16, 16), dtype=np.float32)) * 2 - 1
+    pieces = T.edm_pieces(edm, edm_x)
+    path = os.path.join(OUT, "oracle_vs_reference.npz")
+    np.savez_compressed(path, weights_checksum=np.float64(O.state_checksum(sd)), denoised=dn.numpy(), model_output=mo.numpy(),
+                        edm_x=edm_x.numpy(), **{"edm_" + k: v.numpy() for k, v in pieces.items()})
+    print("oracle_vs_reference size", os.path.getsize(path))
+
+
+def make_reference_surface():
+    """tests/test_host_logic.py: the reference Denoiser's state_dict layout for each config of that test, and the weight-decay
+    split utils.configure_opt makes of the default Denoiser (names of the parameters in its two AdamW groups)."""
+    import dataclasses
+    import json
+
+    T = _test_module("test_host_logic")
+
+    ns = ref_import.load()
+    D = ns.diffusion
+
+    def reference_denoiser(inner):
+        return D.Denoiser(D.DenoiserConfig(D.InnerModelConfig(inner.img_channels, inner.num_steps_conditioning, inner.cond_channels,
+                                                              list(inner.depths), list(inner.channels), list(inner.attn_depths),
+                                                              inner.num_actions), 0.5, 0.3))
+
+    layouts = [{"inner": dataclasses.asdict(inner),
+                "layout": [[k, list(v.shape)] for k, v in reference_denoiser(inner).state_dict().items()]} for inner in T.LAYOUT_CASES]
+    den = reference_denoiser(O.InnerCfg())
+    names = {id(p): n for n, p in den.named_parameters()}
+    opt = ns.utils.configure_opt(den, 1e-4, 1e-2, 1e-8)
+    decay, no_decay = ([names[id(p)] for p in g["params"]] for g in opt.param_groups)
+    path = os.path.join(OUT, "reference_surface.json")
+    with open(path, "w") as f:
+        json.dump({"denoiser_state_dict": layouts, "configure_opt": {"decay": decay, "no_decay": no_decay}}, f, separators=(",", ":"))
+        f.write("\n")
+    print("reference_surface decay / no_decay", len(decay), len(no_decay), "size", os.path.getsize(path))
+
+
+def make_env_host_logic():
+    """tests/test_env_host_logic.py: what the reference's WorldModelEnv and make_env_loop return when driven by that test's fake
+    networks and RNG streams, and its compute_lambda_returns on that test's inputs.  The 401 tensors of the WorldModelEnv run
+    (1.8 MB of incompressible frames) are stored as digests."""
+    T = _test_module("test_env_host_logic")
+
+    ns = ref_import.load()
+    ref_env = ns.envs.world_model_env
+    env = T._run_env(ref_env, ref_env.WorldModelEnvConfig, ns.diffusion.DiffusionSamplerConfig(3))
+    loop = T._run_loop(ns.env_loop.make_env_loop, ref_env, ref_env.WorldModelEnvConfig, ns.diffusion.DiffusionSamplerConfig(3))
+    lam = [ns.actor_critic.compute_lambda_returns(*T.lambda_return_inputs(), 0.985, x) for x in T.LAMBDAS]
+    assert not any(t.is_floating_point() and bool(t.isnan().any()) for t in env)   # digests compare NaNs as equal
+    arrays = {"env_digests": np.array([T.digest(t) for t in env])}
+    for prefix, ts in (("loop", loop), ("lambda_returns", lam)):
+        arrays.update({f"{prefix}_{i:03d}": t.numpy() for i, t in enumerate(ts)})
+    path = os.path.join(OUT, "env_host_logic.npz")
+    np.savez_compressed(path, **arrays)
+    print("env_host_logic tensors", len(arrays), "size", os.path.getsize(path))
+
+
 if __name__ == "__main__":
-    which = sys.argv[1:] or ["inference", "training"]
+    which = sys.argv[1:] or ["inference", "training", "host"]
     named = [w for w in which if w in CASES]   # e.g. `python oracle/make_golden.py denoiser_padded`: only that fixture
     if named:
         main(named)
@@ -292,3 +377,7 @@ if __name__ == "__main__":
     if "training" in which:
         make_denoiser_training()
         make_actor_critic_training()
+    if "host" in which:
+        make_oracle_vs_reference()
+        make_reference_surface()
+        make_env_host_logic()

@@ -1,9 +1,8 @@
 """Test-only helper: import the UNMODIFIED reference (eloialonso/diamond) from /root/reference/src.
 
 ORACLE / TEST INFRASTRUCTURE ONLY.  Nothing in the product path (diamond_b200/) may import this.
-/root/reference does not exist on the GPU box, so this module is only used (a) by
-oracle/make_golden.py to generate tests/golden/*.npz in the build container and (b) by CPU tests
-that are skipped when the reference tree is absent.
+The reference is not part of this repository, so this module is only used by
+oracle/make_golden.py to generate the fixtures under tests/golden/; no test imports it.
 
 The reference needs omegaconf / hydra / gymnasium / ale_py / torcheval at *import* time only
 (utils.py:11, trainer.py:7, envs/env.py:4-6, models/rew_end_model.py:8); none of them is used on the

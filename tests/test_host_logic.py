@@ -1,11 +1,18 @@
 """CPU: host-side mirror of the reference's module surface (no kernel launches)."""
+import dataclasses
+import json
+import os
+
 import pytest
 import torch
 
 from diamond_b200.models.diffusion import (Denoiser, DenoiserConfig, DiffusionSamplerConfig, InnerModelConfig)
 from diamond_b200.models.diffusion.diffusion_sampler import build_sigmas
-from oracle import ref_import
 from oracle import torch_oracle as O
+
+# Denoiser configs whose state_dict layout is pinned to the reference's (tests/golden/reference_surface.json)
+LAYOUT_CASES = [O.InnerCfg(), O.InnerCfg(depths=[1, 2, 1], channels=[32, 64, 32], attn_depths=[0, 0, 1], cond_channels=64,
+                                         num_steps_conditioning=2, num_actions=6)]
 
 
 def _denoiser(inner: O.InnerCfg) -> Denoiser:
@@ -14,20 +21,20 @@ def _denoiser(inner: O.InnerCfg) -> Denoiser:
                                                     inner.num_actions), 0.5, 0.3))
 
 
-@pytest.mark.parametrize("inner", [O.InnerCfg(), O.InnerCfg(depths=[1, 2, 1], channels=[32, 64, 32], attn_depths=[0, 0, 1],
-                                                             cond_channels=64, num_steps_conditioning=2, num_actions=6)])
-def test_state_dict_keys_and_shapes_match_the_reference_layout(inner):
+def _reference_surface(golden_dir):
+    with open(os.path.join(golden_dir, "reference_surface.json")) as f:
+        return json.load(f)
+
+
+@pytest.mark.parametrize("inner", LAYOUT_CASES)
+def test_state_dict_keys_and_shapes_match_the_reference_layout(inner, golden_dir):
     den = _denoiser(inner)
     want = O.inner_model_shapes(inner)
     got = [(k, tuple(v.shape)) for k, v in den.inner_model.state_dict().items()]
     assert got == want
-    if ref_import.available():
-        ns = ref_import.load()
-        D = ns.diffusion
-        ref = D.Denoiser(D.DenoiserConfig(D.InnerModelConfig(inner.img_channels, inner.num_steps_conditioning, inner.cond_channels,
-                                                             list(inner.depths), list(inner.channels), list(inner.attn_depths),
-                                                             inner.num_actions), 0.5, 0.3))
-        assert [(k, tuple(v.shape)) for k, v in ref.state_dict().items()] == [(k, tuple(v.shape)) for k, v in den.state_dict().items()]
+    ref = _reference_surface(golden_dir)["denoiser_state_dict"][LAYOUT_CASES.index(inner)]
+    assert ref["inner"] == dataclasses.asdict(inner)
+    assert [(k, tuple(s)) for k, s in ref["layout"]] == [(k, tuple(v.shape)) for k, v in den.state_dict().items()]
 
 
 def test_default_denoiser_has_the_reference_parameter_count_and_init():
@@ -42,14 +49,15 @@ def test_default_denoiser_has_the_reference_parameter_count_and_init():
     assert torch.allclose(w @ w.t(), torch.eye(64), atol=1e-4)
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference tree absent")
-def test_reference_configure_opt_accepts_the_mirror():
+def test_reference_configure_opt_accepts_the_mirror(golden_dir):
     """utils.configure_opt classifies parameters by isinstance(owner, nn.Conv2d/Linear/GroupNorm/...) and asserts full
-    coverage (utils.py:129-166): expected split for the denoiser is 114 decay / 121 no-decay (SURVEY.md 8b)."""
-    ns = ref_import.load()
+    coverage (utils.py:129-166): its rule (restated by the oracle) splits the mirror exactly as the reference split its own
+    default Denoiser, 114 decay / 121 no-decay (SURVEY.md 8b)."""
     den = _denoiser(O.InnerCfg())
-    opt = ns.utils.configure_opt(den, 1e-4, 1e-2, 1e-8)
-    assert [len(g["params"]) for g in opt.param_groups] == [114, 121]
+    decay, no_decay = O.weight_decay_split(den)
+    ref = _reference_surface(golden_dir)["configure_opt"]
+    assert (decay, no_decay) == (ref["decay"], ref["no_decay"])
+    assert [len(decay), len(no_decay)] == [114, 121]
 
 
 def test_sigma_schedule_matches_reference_values():
