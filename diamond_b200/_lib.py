@@ -122,6 +122,10 @@ SIGNATURES = {
     "dmd_rew_end_set_weights": (_i, [_vp, C.POINTER(_vp), _i, _vp, _vp]),
     "dmd_rew_end_workspace_bytes": (_sz, [_vp, _i]),
     "dmd_rew_end_predict": (_i, [_vp, _i, _i] + [_vp] * 9 + [_vp, _sz, _vp]),
+    "dmd_rew_end_train_workspace_bytes": (_sz, [_vp, _i, _i]),
+    "dmd_rew_end_grad_layout": (C.c_longlong, [_vp, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong), _i]),
+    "dmd_rew_end_forward_train": (_i, [_vp, _i, _i] + [_vp] * 5 + [_vp, _sz, _vp]),
+    "dmd_rew_end_backward": (_i, [_vp, _i, _i, _vp, _vp, _vp, C.c_longlong, _vp, _vp]),
     "dmd_lambda_returns": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, C.c_double, C.c_double, _vp]),
 }
 

@@ -638,6 +638,7 @@ struct Operand {
   bool lazy = false;
   Tens a{}, b{}; bool has_b = false;
   int upsample = 0, mode = 0; const FilmW* film = nullptr; int gamma_idx = 0, beta_idx = 0; bool silu = false, also_raw = false, split = false;
+  bool split_main = false;   // the low part of the main operand as well as of the raw one (a split-fp16 conv reads it)
 };
 
 // backward op list (training).  Parameter-gradient destinations are OFFSETS into the caller's flat gradient buffer.
@@ -668,6 +669,12 @@ struct Rec {
   Operand in1, in2;
 };
 
+// The RewEnd encoder (rew_end_model.py:93-132): U-Net blocks driven by PlanBuilder::build_rew_end.  A training plan built with
+// one of these records the encoder's tape instead of the InnerModel's, and its backward ends in the action-embedding gradient.
+struct EncoderDef {
+  const std::vector<std::vector<ResBlockW>>* blocks; const std::vector<ConvW>* downs; const ConvW* conv_in; int i_actemb;
+};
+
 struct Plan {
   int B = 0, H = 0, W = 0;
   uint8_t* base = nullptr;
@@ -693,6 +700,8 @@ struct Plan {
   long long *film_woff = nullptr, *film_boff = nullptr;   // device tables: flat-gradient offset of every FiLM row
   std::vector<long long> film_woff_h, film_boff_h;
   uint8_t* zero_begin = nullptr; size_t zero_bytes = 0;   // region cleared at the start of every backward (dfilm, sums, amax)
+  Tens enc_out{};                                         // RewEnd encoder output (its .grad receives the LSTM's input gradient)
+  int seq_b = 0, seq_t = 0;                               // RewEnd: (b, t) of the last training forward on this workspace
   // sampler state (NCHW fp32): temporaries only -- the frame stack, the actions and the trajectory are used IN PLACE
   float *s_xc = nullptr, *s_x2 = nullptr, *s_d = nullptr;
   float *sig_all = nullptr, *cemb_all = nullptr, *chid_all = nullptr, *cond_all = nullptr, *film_all = nullptr;  // hoisted conditioning
@@ -854,10 +863,12 @@ struct PlanBuilder {
 
   // mode 0 raw / 1 AdaGroupNorm(film) / 2 GroupNorm(gamma,beta); also_raw: additionally emit the raw operand (skip projection)
   // split: also emit the low fp16 part of the operand that a precise conv will read (raw if also_raw, else the main one)
-  Operand prep(const Tens& a, const Tens* b, int upsample, int mode, const FilmW* film, int gamma_idx, int beta_idx, bool silu, bool also_raw, bool split = false) {
+  Operand prep(const Tens& a, const Tens* b, int upsample, int mode, const FilmW* film, int gamma_idx, int beta_idx, bool silu, bool also_raw,
+               bool split = false, bool split_main = false) {
     Operand o;
     o.a = a; o.has_b = b != nullptr; if (b) o.b = *b;
     o.upsample = upsample; o.mode = mode; o.film = film; o.gamma_idx = gamma_idx; o.beta_idx = beta_idx; o.silu = silu; o.also_raw = also_raw; o.split = split;
+    o.split_main = split_main;
     o.C0 = round_up(a.C, 16); o.C1 = b ? round_up(b->C, 16) : 0;
     o.H = upsample ? 2 * a.H : a.H; o.W = upsample ? 2 * a.W : a.W;
     // small problems (at most one tile per SM) may leave the transform to the consuming conv (conv_fused_kernel, DMD_FUSE_SMALL=1;
@@ -888,7 +899,7 @@ struct PlanBuilder {
     if (b) { o.n1 = scratch(); d.dst1 = o.n1; }
     if (o.also_raw) { o.r0 = scratch(); d.dst_raw0 = o.r0; if (b) { o.r1 = scratch(); d.dst_raw1 = o.r1; } }
     if (o.split && o.also_raw) { o.rl0 = scratch(); d.dst_raw_lo0 = o.rl0; if (b) { o.rl1 = scratch(); d.dst_raw_lo1 = o.rl1; } }
-    if (o.split && !o.also_raw) { o.nl0 = scratch(); d.dst_lo0 = o.nl0; }
+    if ((o.split && !o.also_raw) || o.split_main) { o.nl0 = scratch(); d.dst_lo0 = o.nl0; }
     Op op; op.kind = OP_PREP;
     if (prep_fill(&d, &op.prep, &op.prep_nsrc)) { err = 1; return; }
     o.op = (int)pl->ops.size();
@@ -968,6 +979,7 @@ struct PlanBuilder {
     d.residual = resid ? (resid->data ? resid->data : (const float*)1) : nullptr; d.out = out.data ? out.data : (float*)1;
     d.out_stats = out_stats ? (out.stats ? out.stats : (double*)1) : nullptr; d.out_gs = out.gs;
     if (cw.precise && (!d.src0_lo || (in.C1 && !d.src1_lo))) { fail("plan: precise conv without low operand parts"); err = 1; return; }
+    if (cw.precise && !raw && in.C1) { fail("plan: a split-fp16 conv of a normalised concat is not built"); err = 1; return; }
     if (in.C0 + in.C1 != cw.Cin) { fail("plan: operand channels %d+%d do not match the packed weights (%d)", in.C0, in.C1, cw.Cin); err = 1; return; }
     Op op; op.kind = OP_CONV;
     if (conv_fill(&d, &op.conv, &op.smem, &op.cols)) { err = 1; return; }
@@ -977,10 +989,10 @@ struct PlanBuilder {
   // ResBlock.forward (blocks.py:141-147)
   Tens resblock(const ResBlockW& rb, const Tens& x, const Tens* skip) {
     const int H = x.H, W = x.W;
-    Operand in1 = prep(x, skip, 0, 1, &rb.n1, 0, 0, true, rb.has_proj != 0, rb.has_proj != 0);
+    Operand in1 = prep(x, skip, 0, 1, &rb.n1, 0, 0, true, rb.has_proj != 0, rb.has_proj != 0, rb.c1.precise != 0);
     Tens t = tensor(rb.cout, H, W, true, false);   // its gradient lives in a temporary
     conv(rb.c1, in1, false, 1, nullptr, t, true);
-    Operand in2 = prep(t, nullptr, 0, 1, &rb.n2, 0, 0, true, false);
+    Operand in2 = prep(t, nullptr, 0, 1, &rb.n2, 0, 0, true, false, rb.c2.precise != 0);
     Tens o = tensor(rb.cout, H, W, true);
     // x + r: r is the block input itself, or proj(input) fused into conv2's accumulator (no r tensor, no extra launch)
     if (rb.has_proj) conv(rb.c2, in2, false, 1, nullptr, o, true, &rb.proj, &in1);
@@ -1014,11 +1026,17 @@ struct PlanBuilder {
     pl->film = (float*)bump->take((size_t)B * h->film_rows * 4);
     Tens xin{pl->xin, nullptr, pl->CP_in, H, W, 8};
     Tens x = tensor(c.channels[0], H, W, true);
-    { Operand in0 = prep(xin, nullptr, 0, 0, nullptr, 0, 0, false, false, true); conv(conv_in, in0, false, 1, nullptr, x, true); }
+    {
+      Operand in0 = prep(xin, nullptr, 0, 0, nullptr, 0, 0, false, false, true);
+      conv(conv_in, in0, false, 1, nullptr, x, true);
+      Rec rec; rec.kind = R_CONVIN; rec.cw = &conv_in; rec.x = xin; rec.o = x; rec.in1 = in0; record(rec);
+    }
     for (int i = 0; i <= L; ++i) {
       if (i > 0 && i < L) {
         Tens xd = tensor(c.channels[i - 1], x.H / 2, x.W / 2, true);
-        { Operand ind = prep(x, nullptr, 0, 0, nullptr, 0, 0, false, false); conv(downs[i], ind, false, 2, nullptr, xd, true); }
+        Operand ind = prep(x, nullptr, 0, 0, nullptr, 0, 0, false, false, downs[i].precise != 0);
+        conv(downs[i], ind, false, 2, nullptr, xd, true);
+        Rec rec; rec.kind = R_DOWN; rec.cw = &downs[i]; rec.x = x; rec.o = xd; rec.in1 = ind; record(rec);
         x = xd;
       }
       for (auto& rb : blocks[i]) x = resblock(rb, x, nullptr);
@@ -1144,7 +1162,7 @@ int make_plan(dmd_denoiser* h, Plan* pl, int B, int H, int W, uint8_t* base, siz
 // loss scale; "first writer assigns, later writers accumulate" is decided here at plan time (ginit), so no gradient
 // buffer needs a memset.  Forward conv inputs (the PLC16 operands) are not kept: the forward prep launch is replayed.
 struct BwdBuilder {
-  dmd_denoiser* h; Plan* pl; Bump* bump; int err = 0;
+  dmd_denoiser* h; Plan* pl; Bump* bump; const EncoderDef* enc = nullptr; int err = 0;
   std::vector<char> ginit;
 
   const float* P(int idx) const { return h->ptrs.empty() ? nullptr : h->ptrs[idx]; }
@@ -1304,7 +1322,7 @@ struct BwdBuilder {
       }
       if (err) return 1;
     }
-    // ---- conditioning path (inner_model.py:45; blocks.py:39): FiLM linears, cond_proj MLP, action embedding
+    // ---- conditioning path (inner_model.py:45; blocks.py:39): FiLM linears, then cond_proj MLP and action embedding
     const dmd_denoiser_config& c = h->cfg;
     const int CC = c.cond_channels, R = h->film_rows;
     { BOp b; b.kind = B_FILMW; push(b); }
@@ -1322,6 +1340,10 @@ struct BwdBuilder {
       int splits = R / 256; if (splits > 32) splits = 32; if (splits > fit) splits = (int)fit;
       if (splits > 1) pl->bops.back().chunks = splits;
     }
+    if (enc) {   // RewEnd: cond = act_emb(act) (rew_end_model.py:51), one embedding row per encoder row
+      BOp b; b.kind = B_EMB; b.src = pl->dcond; b.goff = h->goff[enc->i_actemb]; push(b);
+      return err;
+    }
     sgemm(pl->dcond, 1, CC, pl->chid, CC, 1, nullptr, h->goff[h->i_cp2w], CC, CC, CC, B, 1, 1);  // dW2 += dcond^T h
     colsum(pl->dcond, B, CC, CC, h->i_cp2b);
     sgemm(pl->dcond, CC, 1, P(h->i_cp2w), CC, 1, pl->dh, -1, CC, B, CC, CC, 0, 0);               // dh = dcond W2
@@ -1335,16 +1357,20 @@ struct BwdBuilder {
   }
 };
 
-// training workspace = forward plan (with gradient buffers) + backward temporaries
-int make_train_plan(dmd_denoiser* h, Plan* pl, int B, int H, int W, uint8_t* base, size_t* total) {
+// training workspace = forward plan (with gradient buffers) + backward temporaries.  enc: the RewEnd encoder instead of
+// the InnerModel (its forward records the encoder's tape and its backward ends in the action embedding)
+int make_train_plan(dmd_denoiser* h, Plan* pl, int B, int H, int W, uint8_t* base, size_t* total, const EncoderDef* enc = nullptr) {
   pl->train = true; pl->n_grad_tensors = 0; pl->tape.clear();
   pl->B = B; pl->H = H; pl->W = W; pl->ops.clear(); pl->bops.clear();
+  auto build_fwd = [&](PlanBuilder& pb, Plan* p) {
+    return enc ? pb.build_rew_end(*enc->blocks, *enc->downs, *enc->conv_in, &p->enc_out) : pb.build();
+  };
   Bump b0{nullptr}, s0{nullptr};
-  { Plan tmp; tmp.train = true; tmp.B = B; tmp.H = H; tmp.W = W; PlanBuilder pb{h, &tmp, &b0, &s0}; if (pb.build()) return 1; }
+  { Plan tmp; tmp.train = true; tmp.B = B; tmp.H = H; tmp.W = W; PlanBuilder pb{h, &tmp, &b0, &s0}; if (build_fwd(pb, &tmp)) return 1; }
   const size_t stats_bytes = (s0.off + 255) & ~(size_t)255;
   Bump sb{base}, bb{base ? base + stats_bytes : nullptr};
   if (base) { pl->base = base; pl->stats = (double*)base; pl->stats_bytes = stats_bytes; }
-  if (base) { PlanBuilder pb{h, pl, &bb, &sb}; if (pb.build()) return 1; } else bb.off = b0.off;
+  if (base) { PlanBuilder pb{h, pl, &bb, &sb}; if (build_fwd(pb, pl)) return 1; } else bb.off = b0.off;
   // backward temporaries
   const dmd_denoiser_config& c = h->cfg;
   int cmax = 16;
@@ -1353,7 +1379,7 @@ int make_train_plan(dmd_denoiser* h, Plan* pl, int B, int H, int W, uint8_t* bas
   pl->tA = (float*)bb.take(act_bytes); pl->tB = (float*)bb.take(act_bytes); pl->tC = (float*)bb.take(act_bytes);
   const size_t op_bytes = plc16_bytes(B, H, W, cmax);
   pl->gyA = (uint8_t*)bb.take(op_bytes); pl->gyB = (uint8_t*)bb.take(op_bytes);
-  pl->gF = (float*)bb.take((size_t)B * H * W * 8 * 4);
+  if (!enc) pl->gF = (float*)bb.take((size_t)B * H * W * 8 * 4);
   if (init_kernels()) return 1;
   pl->partial = (float*)bb.take(wgrad_partial_bytes(g_num_sms));
   const int CC = c.cond_channels;
@@ -1370,7 +1396,7 @@ int make_train_plan(dmd_denoiser* h, Plan* pl, int B, int H, int W, uint8_t* bas
   if (total) *total = stats_bytes + bb.off + 512;
   if (!base) return 0;
   pl->bytes = stats_bytes + bb.off;
-  BwdBuilder bw{h, pl, &bb};
+  BwdBuilder bw{h, pl, &bb, enc};
   if (bw.build()) return 1;
   // flat-gradient offsets of every FiLM row (weights) / element (biases)
   pl->film_woff_h.assign(h->film_rows, 0); pl->film_boff_h.assign(h->film_rows, 0);
@@ -1378,6 +1404,10 @@ int make_train_plan(dmd_denoiser* h, Plan* pl, int B, int H, int W, uint8_t* bas
     for (int r = 0; r < 2 * f.C; ++r) { pl->film_woff_h[f.off + r] = h->goff[f.w_idx] + (long long)r * CC; pl->film_boff_h[f.off + r] = h->goff[f.b_idx] + r; }
   };
   auto fill_rb = [&](const ResBlockW& r) { fill_film(r.n1); fill_film(r.n2); };
+  if (enc) {
+    for (auto& lv : *enc->blocks) for (auto& r : lv) fill_rb(r);
+    return 0;
+  }
   for (auto& lv : h->d_blocks) for (auto& r : lv) fill_rb(r);
   for (auto& lv : h->u_blocks) for (auto& r : lv) fill_rb(r);
   for (auto& r : h->mid) fill_rb(r);
@@ -1539,11 +1569,12 @@ Plan* find_train_plan(dmd_denoiser* h, int B, int H, int W, void* ws) {
   return nullptr;
 }
 
-int ensure_train_plan(dmd_denoiser* h, int B, int H, int W, void* ws, size_t ws_bytes, cudaStream_t st, Plan** out) {
+int ensure_train_plan(dmd_denoiser* h, int B, int H, int W, void* ws, size_t ws_bytes, cudaStream_t st, Plan** out,
+                      const EncoderDef* enc = nullptr) {
   DMD_CHECK(!h->ptrs.empty() && h->packed, "denoiser: call dmd_denoiser_set_weights first");
   if ((*out = find_train_plan(h, B, H, W, ws)) != nullptr) return 0;
   size_t need = 0;
-  { Plan tmp; if (make_train_plan(h, &tmp, B, H, W, nullptr, &need)) return 1; }
+  { Plan tmp; if (make_train_plan(h, &tmp, B, H, W, nullptr, &need, enc)) return 1; }
   DMD_CHECK(ws && ws_bytes >= need, "denoiser: training workspace too small (%zu < %zu)", ws_bytes, need);
   DMD_CHECK(((uintptr_t)ws & 255) == 0, "denoiser: workspace must be 256-byte aligned");
   // a plan bound to the same workspace with another shape is stale; keep at most 8 plans
@@ -1551,7 +1582,7 @@ int ensure_train_plan(dmd_denoiser* h, int B, int H, int W, void* ws, size_t ws_
     if (h->tplans[i]->base == (uint8_t*)ws) h->tplans.erase(h->tplans.begin() + i); else ++i;
   if (h->tplans.size() >= 8) h->tplans.erase(h->tplans.begin());
   std::unique_ptr<Plan> pl(new Plan());
-  if (make_train_plan(h, pl.get(), B, H, W, (uint8_t*)ws, nullptr)) return 1;
+  if (make_train_plan(h, pl.get(), B, H, W, (uint8_t*)ws, nullptr, enc)) return 1;
   DMD_CUDA(cudaMemcpyAsync(pl->film_woff, pl->film_woff_h.data(), pl->film_woff_h.size() * 8, cudaMemcpyHostToDevice, st));
   DMD_CUDA(cudaMemcpyAsync(pl->film_boff, pl->film_boff_h.data(), pl->film_boff_h.size() * 8, cudaMemcpyHostToDevice, st));
   *out = pl.get();
@@ -1559,20 +1590,11 @@ int ensure_train_plan(dmd_denoiser* h, int B, int H, int W, void* ws, size_t ws_
   return 0;
 }
 
-int run_backward(dmd_denoiser* h, Plan& pl, const float* grad_out, float* grads, cudaStream_t st) {
+// the backward op list of a training plan; the caller has cleared the zeroed region and set the loss scale in pl.scale
+int run_bops(dmd_denoiser* h, Plan& pl, float* grads, cudaStream_t st) {
   const dmd_denoiser_config& c = h->cfg;
-  const int B = pl.B, HW = pl.H * pl.W, CC = c.cond_channels;
+  const int B = pl.B, CC = c.cond_channels;
   const float* inv = pl.scale + 1;
-  DMD_CUDA(cudaMemsetAsync(grads, 0, (size_t)h->grad_total * 4, st));
-  DMD_CUDA(cudaMemsetAsync(pl.zero_begin, 0, pl.zero_bytes, st));
-  // loss scale from the incoming gradient, then the scaled NHWC gradient of the model output
-  const long long n_out = (long long)B * c.img_channels * HW;
-  absmax_kernel<<<(int)std::min<long long>((n_out + 255) / 256, 1184), 256, 0, st>>>(grad_out, pl.amax, n_out);
-  DMD_LAUNCH_OK();
-  loss_scale_kernel<<<1, 1, 0, st>>>(pl.amax, pl.scale);
-  DMD_LAUNCH_OK();
-  nchw_to_nhwc_scaled_kernel<<<dim3((HW + 255) / 256, B), 256, 0, st>>>(grad_out, pl.gF, pl.scale, c.img_channels, 8, HW);
-  DMD_LAUNCH_OK();
   for (const BOp& b : pl.bops) {
     switch (b.kind) {
       case B_PREP: if (prep_launch(b.prep, b.prep_nsrc, st)) return 1; break;
@@ -1638,6 +1660,22 @@ int run_backward(dmd_denoiser* h, Plan& pl, const float* grad_out, float* grads,
     }
   }
   return 0;
+}
+
+int run_backward(dmd_denoiser* h, Plan& pl, const float* grad_out, float* grads, cudaStream_t st) {
+  const dmd_denoiser_config& c = h->cfg;
+  const int B = pl.B, HW = pl.H * pl.W;
+  DMD_CUDA(cudaMemsetAsync(grads, 0, (size_t)h->grad_total * 4, st));
+  DMD_CUDA(cudaMemsetAsync(pl.zero_begin, 0, pl.zero_bytes, st));
+  // loss scale from the incoming gradient, then the scaled NHWC gradient of the model output
+  const long long n_out = (long long)B * c.img_channels * HW;
+  absmax_kernel<<<(int)std::min<long long>((n_out + 255) / 256, 1184), 256, 0, st>>>(grad_out, pl.amax, n_out);
+  DMD_LAUNCH_OK();
+  loss_scale_kernel<<<1, 1, 0, st>>>(pl.amax, pl.scale);
+  DMD_LAUNCH_OK();
+  nchw_to_nhwc_scaled_kernel<<<dim3((HW + 255) / 256, B), 256, 0, st>>>(grad_out, pl.gF, pl.scale, c.img_channels, 8, HW);
+  DMD_LAUNCH_OK();
+  return run_bops(h, pl, grads, st);
 }
 
 }  // namespace
@@ -2266,13 +2304,20 @@ struct dmd_rew_end {
   Tens feat;
   int planB = 0; void* plan_ws = nullptr;
   float *x_gates = nullptr, *y = nullptr, *hid = nullptr, *logits_tm = nullptr, *hc[2] = {nullptr, nullptr};
+  // Training plans (core.tplans, apart from the inference plan core.plan) run the encoder's ResBlock and Downsample convs in
+  // split-fp16: with single-fp16 operands the forward's rounding reaches the LSTM / head weight gradients (emulated: 1.3e-3
+  // whole-gradient error vs fp32; split: 3.3e-4, DESIGN.md section 2).  Copies of those convs with their own split packs;
+  // the backward-data packs are shared.
+  std::vector<std::vector<ResBlockW>> tblocks;
+  std::vector<ConvW> tdowns;
+  EncoderDef enc{};
 };
 
 namespace {
 
 __global__ void pack_rew_end_input_kernel(const float* __restrict__ obs, const float* __restrict__ next_obs, const int64_t* __restrict__ act,
                                           const float* __restrict__ act_emb, float* __restrict__ xin, float* __restrict__ cond, int b, int t,
-                                          int C, int CP, int HW, int CC, int num_actions) {
+                                          int C, int CP, int HW, int CC, int num_actions, int64_t* __restrict__ act_tm = nullptr) {
   // row r = k * b + n (time-major)  <-  obs[n][k], next_obs[n][k], act[n][k]
   const int r = blockIdx.y, k = r / b, n = r - k * b;
   const size_t src = ((size_t)n * t + k) * C * HW;
@@ -2281,6 +2326,7 @@ __global__ void pack_rew_end_input_kernel(const float* __restrict__ obs, const f
     long long a = act[(size_t)n * t + k];
     a = a < 0 ? 0 : (a >= num_actions ? num_actions - 1 : a);
     for (int j = threadIdx.x; j < CC; j += blockDim.x) cond[(size_t)r * CC + j] = act_emb[(size_t)a * CC + j];
+    if (act_tm && threadIdx.x == 0) act_tm[r] = a;   // training: the embedding backward reads the actions in row order
   }
   if (pix >= HW) return;
   float* o = xin + ((size_t)r * HW + pix) * CP;
@@ -2299,6 +2345,26 @@ __global__ void split_logits_kernel(const float* __restrict__ tm, float* __restr
   const float* s = tm + ((size_t)k * b + n) * 5;
   rew[(size_t)i * 3] = s[0]; rew[(size_t)i * 3 + 1] = s[1]; rew[(size_t)i * 3 + 2] = s[2];
   end[(size_t)i * 2] = s[3]; end[(size_t)i * 2 + 1] = s[4];
+}
+// the adjoint of split_logits_kernel: g_rew [b][t][3], g_end [b][t][2] -> g_tm [t*b][5] (time-major)
+__global__ void merge_logits_grad_kernel(const float* __restrict__ g_rew, const float* __restrict__ g_end, float* __restrict__ g_tm, int b, int t) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= b * t) return;
+  const int n = i / t, k = i - n * t;
+  float* d = g_tm + ((size_t)k * b + n) * 5;
+  d[0] = g_rew[(size_t)i * 3]; d[1] = g_rew[(size_t)i * 3 + 1]; d[2] = g_rew[(size_t)i * 3 + 2];
+  d[3] = g_end[(size_t)i * 2]; d[4] = g_end[(size_t)i * 2 + 1];
+}
+
+// the encoder's forward op list (inference and training plans alike)
+int run_encoder_ops(const Plan& pl, cudaStream_t st) {
+  for (const Op& op : pl.ops) {
+    if (op.kind == OP_CONV) { if (conv_launch(op.conv, op.smem, op.cols, st)) return 1; }
+    else if (op.kind == OP_PREP) { if (prep_launch(op.prep, op.prep_nsrc, st)) return 1; }
+    else if (op.kind == OP_FUSED) { if (fused_launch(op.fused, op.smem, op.cols, st)) return 1; }
+    else { if (attn_launch(op.attn, pl.B, st)) return 1; }
+  }
+  return 0;
 }
 
 int rew_end_layout(dmd_rew_end* h, int B, int H, int W, uint8_t* base, size_t* total) {
@@ -2361,7 +2427,20 @@ extern "C" dmd_rew_end* dmd_rew_end_create(const dmd_rew_end_config* cfg) {
   h->i_wih = w.next(4 * D * K); h->i_whh = w.next(4 * D * D); h->i_bih = w.next(4 * D); h->i_bhh = w.next(4 * D);
   h->i_h0w = w.next(D * D); h->i_h0b = w.next(D); h->i_h2w = w.next(5 * D);
   core->n_tensors = w.idx;
+  core->goff.assign(core->n_tensors, 0);
+  core->grad_total = 0;
+  for (int i = 0; i < core->n_tensors; ++i) { core->goff[i] = core->grad_total; core->grad_total += (core->numel[i] + 3) & ~3ll; }  // 16-byte aligned slices
   size_t pk = w.pk;
+  auto split_copy = [&](ConvW c) {
+    c.precise = 1; c.trs = 0; c.pk_off = pk;
+    pk += (size_t)c.taps * c.Cin * c.CoutPad * 2 * 3; pk = (pk + 255) & ~(size_t)255;
+    return c;
+  };
+  h->tblocks = h->blocks;
+  for (auto& lv : h->tblocks) for (auto& r : lv) { r.c1 = split_copy(r.c1); r.c2 = split_copy(r.c2); }
+  h->tdowns = h->downs;
+  for (int i = 1; i < L; ++i) h->tdowns[i] = split_copy(h->downs[i]);
+  h->enc = EncoderDef{&h->tblocks, &h->tdowns, &h->conv_in, h->i_actemb};
   core->film_w_off = pk; pk += (size_t)core->film_rows * cfg->cond_channels * 4; pk = (pk + 255) & ~(size_t)255;
   core->film_b_off = pk; pk += (size_t)core->film_rows * 4; pk = (pk + 255) & ~(size_t)255;
   core->packed_bytes = pk;
@@ -2376,12 +2455,20 @@ extern "C" int dmd_rew_end_set_weights(dmd_rew_end* h, const float* const* ptrs_
   dmd_denoiser* core = &h->core;
   DMD_CHECK(n_ptrs == core->n_tensors, "rew_end set_weights: expected %d tensors (RewEndModel.state_dict order), got %d", core->n_tensors, n_ptrs);
   cudaStream_t st = (cudaStream_t)stream;
+  // training plans bake parameter and packed-weight addresses in: drop them when these move
+  const bool moved = core->packed != (uint8_t*)packed || core->ptrs.empty() || memcmp(core->ptrs.data(), ptrs_host, sizeof(float*) * n_ptrs) != 0;
+  if (moved) core->tplans.clear();
   core->ptrs.assign(ptrs_host, ptrs_host + n_ptrs);
   core->packed = (uint8_t*)packed;
   h->planB = 0;
   if (pack_one(core, h->conv_in, st)) return 1;
   for (auto& lv : h->blocks) for (auto& r : lv) if (pack_rb(core, r, st)) return 1;
   for (int i = 1; i < h->cfg.num_levels; ++i) if (pack_one(core, h->downs[i], st)) return 1;
+  auto pack_split = [&](const ConvW& c) {   // the training copies' forward packs (their backward-data packs are the ones above)
+    return dmd_pack_conv_weight(core->ptrs[c.w_idx], core->packed + c.pk_off, c.Cout, c.CoutPad, c.CinReal, c.Cin, c.taps, c.c0_real, c.c0_store, 1, st);
+  };
+  for (auto& lv : h->tblocks) for (auto& r : lv) if (pack_split(r.c1) || pack_split(r.c2)) return 1;
+  for (int i = 1; i < h->cfg.num_levels; ++i) if (pack_split(h->tdowns[i])) return 1;
   return 0;
 }
 
@@ -2419,12 +2506,7 @@ extern "C" int dmd_rew_end_predict(dmd_rew_end* h, int b, int t, const float* ob
   DMD_LAUNCH_OK();
   if (linear_launch(pl.cond, (const float*)(core->packed + core->film_w_off), (const float*)(core->packed + core->film_b_off), pl.film,
                     rows, CC, core->film_rows, 0, st)) return 1;
-  for (const Op& op : pl.ops) {
-    if (op.kind == OP_CONV) { if (conv_launch(op.conv, op.smem, op.cols, st)) return 1; }
-    else if (op.kind == OP_PREP) { if (prep_launch(op.prep, op.prep_nsrc, st)) return 1; }
-    else if (op.kind == OP_FUSED) { if (fused_launch(op.fused, op.smem, op.cols, st)) return 1; }
-    else { if (attn_launch(op.attn, pl.B, st)) return 1; }
-  }
+  if (run_encoder_ops(pl, st)) return 1;
   // LSTM over time (torch.nn.LSTM, gate order i f g o), rows of step k are the contiguous block [k*b, (k+1)*b)
   const int K = h->feat_c * h->feat_hw;
   const float* hprev = hx_in; const float* cprev = cx_in;
@@ -2446,4 +2528,184 @@ extern "C" int dmd_rew_end_predict(dmd_rew_end* h, int b, int t, const float* ob
   split_logits_kernel<<<(rows + 127) / 128, 128, 0, st>>>(h->logits_tm, logits_rew, logits_end, b, t);
   DMD_LAUNCH_OK();
   return 0;
+}
+
+// ---------------------------------------------------------------------------------------------- reward / termination training
+// RewEndModel.forward under autograd (rew_end_model.py:57-90, trainer.py:349-388).  dmd_rew_end_forward_train runs the
+// encoder on a training plan of its own (core.tplans: a later predict_rew_end keeps its inference plan) and keeps every
+// activation: the encoder tape, all t steps of LSTM gates and cell states, and the head input.  dmd_rew_end_backward
+// then runs the head backward, BPTT through the LSTM (fp32), and the encoder backward under one power-of-two loss scale.
+// Workspace = [encoder training plan][RewEndTrain buffers below]; rows are time-major (r = k * b + n).
+namespace {
+
+struct RewEndTrain {
+  int64_t* act_tm; float *gates, *cells, *y, *hid, *logits_tm, *zeros;                 // forward
+  float *g_logits, *hpre, *g_pre, *g_hid, *g_y, *dgates, *g_c[2], *x_flat, *g_xflat;     // backward
+  size_t bytes;
+};
+
+void rew_end_train_layout(const dmd_rew_end* h, int b, int t, uint8_t* base, RewEndTrain* o) {
+  Bump bb{base};
+  const size_t rows = (size_t)b * t, D = h->cfg.lstm_dim, K = (size_t)h->feat_c * h->feat_hw;
+  o->act_tm = (int64_t*)bb.take(rows * 8);
+  o->gates = (float*)bb.take(rows * 4 * D * 4); o->cells = (float*)bb.take(rows * D * 4);
+  o->y = (float*)bb.take(rows * D * 4); o->hid = (float*)bb.take(rows * D * 4);
+  o->logits_tm = (float*)bb.take(rows * 5 * 4); o->zeros = (float*)bb.take((size_t)b * D * 4);
+  o->g_logits = (float*)bb.take(rows * 5 * 4);
+  o->hpre = (float*)bb.take(rows * D * 4); o->g_pre = (float*)bb.take(rows * D * 4);
+  o->g_hid = (float*)bb.take(rows * D * 4); o->g_y = (float*)bb.take(rows * D * 4);
+  o->dgates = (float*)bb.take(rows * 4 * D * 4);
+  o->g_c[0] = (float*)bb.take((size_t)b * D * 4); o->g_c[1] = (float*)bb.take((size_t)b * D * 4);
+  o->x_flat = (float*)bb.take(rows * K * 4); o->g_xflat = (float*)bb.take(rows * K * 4);
+  o->bytes = bb.off + 256;
+}
+
+// bytes of the encoder training plan (its buffers start the workspace); 0 with dmd_last_error set when it cannot be built
+size_t rew_end_plan_bytes(dmd_rew_end* h, int rows) {
+  Plan tmp; size_t need = 0;
+  const int S = h->cfg.img_size;
+  if (make_train_plan(&h->core, &tmp, rows, S, S, nullptr, &need, &h->enc)) return 0;
+  return (need + 255) & ~(size_t)255;
+}
+
+int rew_end_check_bt(int b, int t, const char* who) {
+  DMD_CHECK(b > 0 && t > 0, "%s: b and t must be positive (got b=%d t=%d)", who, b, t);
+  DMD_CHECK((long long)b * t < (1ll << 24), "%s: b * t = %lld rows is too many", who, (long long)b * t);
+  return 0;
+}
+
+}  // namespace
+
+extern "C" size_t dmd_rew_end_train_workspace_bytes(dmd_rew_end* h, int b, int t) {
+  if (!h) { fail("rew_end train_workspace_bytes: null handle"); return 0; }
+  if (rew_end_check_bt(b, t, "rew_end train_workspace_bytes")) return 0;
+  const size_t plan = rew_end_plan_bytes(h, b * t);
+  if (!plan) return 0;
+  RewEndTrain r; rew_end_train_layout(h, b, t, nullptr, &r);
+  return plan + r.bytes;
+}
+
+extern "C" long long dmd_rew_end_grad_layout(const dmd_rew_end* h, long long* offsets, long long* numels, int n) {
+  if (!h || n != h->core.n_tensors) { fail("rew_end grad_layout: expected %d entries", h ? h->core.n_tensors : 0); return -1; }
+  for (int i = 0; i < n; ++i) { if (offsets) offsets[i] = h->core.goff[i]; if (numels) numels[i] = h->core.numel[i]; }
+  return h->core.grad_total;
+}
+
+extern "C" int dmd_rew_end_forward_train(dmd_rew_end* h, int b, int t, const float* obs, const float* next_obs, const int64_t* act,
+                                         float* logits_rew, float* logits_end, void* workspace, size_t workspace_bytes, void* stream) {
+  DMD_CHECK(h && obs && next_obs && act && logits_rew && logits_end && workspace, "rew_end forward_train: null argument");
+  if (rew_end_check_bt(b, t, "rew_end forward_train")) return 1;
+  dmd_denoiser* core = &h->core;
+  DMD_CHECK(!core->ptrs.empty() && core->packed, "rew_end forward_train: call dmd_rew_end_set_weights first");
+  DMD_CHECK(((uintptr_t)workspace & 255) == 0, "rew_end forward_train: workspace must be 256-byte aligned");
+  const dmd_rew_end_config& c = h->cfg;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int rows = b * t, S = c.img_size, HW = S * S, D = c.lstm_dim, CC = c.cond_channels, K = h->feat_c * h->feat_hw;
+  const size_t plan_bytes = rew_end_plan_bytes(h, rows);
+  if (!plan_bytes) return 1;
+  RewEndTrain r; rew_end_train_layout(h, b, t, nullptr, &r);
+  DMD_CHECK(workspace_bytes >= plan_bytes + r.bytes, "rew_end forward_train: workspace too small (%zu < %zu)", workspace_bytes, plan_bytes + r.bytes);
+  Plan* pl = nullptr;
+  if (ensure_train_plan(core, rows, S, S, workspace, plan_bytes, st, &pl, &h->enc)) return 1;
+  rew_end_train_layout(h, b, t, (uint8_t*)workspace + plan_bytes, &r);
+  pl->seq_b = 0; pl->seq_t = 0;   // set again once the forward has been issued
+  pl->t_act = r.act_tm;
+  DMD_CUDA(cudaMemsetAsync(pl->stats, 0, pl->stats_bytes, st));
+  pack_rew_end_input_kernel<<<dim3((HW + 255) / 256, rows), 256, 0, st>>>(obs, next_obs, act, core->ptrs[h->i_actemb], pl->xin, pl->cond, b, t,
+                                                                          c.img_channels, pl->CP_in, HW, CC, c.num_actions, r.act_tm);
+  DMD_LAUNCH_OK();
+  if (linear_launch(pl->cond, (const float*)(core->packed + core->film_w_off), (const float*)(core->packed + core->film_b_off), pl->film,
+                    rows, CC, core->film_rows, 0, st)) return 1;
+  if (run_encoder_ops(*pl, st)) return 1;
+  // LSTM from a zero state (rew_end_model.py:53); the input projection of all t steps at once, then the recurrence.  Gates
+  // (pre-activations) and cell states of every step stay for the backward.
+  if (linear_launch(pl->enc_out.data, core->ptrs[h->i_wih], core->ptrs[h->i_bih], r.gates, rows, K, 4 * D, 0, st, 0, h->feat_hw)) return 1;
+  DMD_CUDA(cudaMemsetAsync(r.zeros, 0, (size_t)b * D * 4, st));
+  for (int k = 0; k < t; ++k) {
+    float* gk = r.gates + (size_t)k * b * 4 * D;
+    const float* hprev = k ? r.y + (size_t)(k - 1) * b * D : r.zeros;
+    const float* cprev = k ? r.cells + (size_t)(k - 1) * b * D : r.zeros;
+    if (linear_launch(hprev, core->ptrs[h->i_whh], core->ptrs[h->i_bhh], gk, b, D, 4 * D, 0, st, 1, 0)) return 1;
+    lstm_gates_kernel<<<(b * D + 255) / 256, 256, 0, st>>>(gk, cprev, r.y + (size_t)k * b * D, r.cells + (size_t)k * b * D, b, D);
+    DMD_LAUNCH_OK();
+  }
+  if (linear_launch(r.y, core->ptrs[h->i_h0w], core->ptrs[h->i_h0b], r.hid, rows, D, D, 1, st)) return 1;
+  if (linear_launch(r.hid, core->ptrs[h->i_h2w], nullptr, r.logits_tm, rows, D, 5, 0, st)) return 1;
+  split_logits_kernel<<<(rows + 127) / 128, 128, 0, st>>>(r.logits_tm, logits_rew, logits_end, b, t);
+  DMD_LAUNCH_OK();
+  pl->seq_b = b; pl->seq_t = t;
+  return 0;
+}
+
+// g_logits_rew (b, t, 3), g_logits_end (b, t, 2): dL/dlogits.  Writes (assigns) every parameter gradient into `grads`.
+extern "C" int dmd_rew_end_backward(dmd_rew_end* h, int b, int t, const float* g_logits_rew, const float* g_logits_end, float* grads,
+                                    long long grads_numel, void* workspace, void* stream) {
+  DMD_CHECK(h && g_logits_rew && g_logits_end && grads && workspace, "rew_end backward: null argument");
+  if (rew_end_check_bt(b, t, "rew_end backward")) return 1;
+  dmd_denoiser* core = &h->core;
+  const int rows = b * t, S = h->cfg.img_size, D = h->cfg.lstm_dim, K = h->feat_c * h->feat_hw;
+  Plan* plp = find_train_plan(core, rows, S, S, workspace);
+  DMD_CHECK(plp && plp->train && plp->seq_b == b && plp->seq_t == t,
+            "rew_end backward: no matching dmd_rew_end_forward_train on this workspace (b=%d t=%d)", b, t);
+  Plan& pl = *plp;
+  DMD_CHECK(grads_numel >= core->grad_total, "rew_end backward: gradient buffer too small (%lld < %lld floats)", grads_numel, core->grad_total);
+  DMD_CHECK(((uintptr_t)grads & 15) == 0, "rew_end backward: gradient buffer must be 16-byte aligned");
+  cudaStream_t st = (cudaStream_t)stream;
+  RewEndTrain r; rew_end_train_layout(h, b, t, (uint8_t*)workspace + rew_end_plan_bytes(h, rows), &r);
+  auto G = [&](int idx) { return grads + core->goff[idx]; };
+  auto W = [&](int idx) { return core->ptrs[idx]; };
+  // C (+)= A B with A(m, k) = A[m * sam + k * sak], B(k, n) = B[k * sbk + n * sbn]  (fp32)
+  auto sgemm = [&](const float* A, long long sam, long long sak, const float* Bm, long long sbk, long long sbn, float* C, long long ldc,
+                   int M, int N, int Kd, int acc) -> int {
+    sgemm_kernel<<<dim3((N + 63) / 64, (M + 63) / 64), 256, 0, st>>>(A, sam, sak, Bm, sbk, sbn, C, ldc, M, N, Kd, nullptr, acc);
+    DMD_LAUNCH_OK();
+    return 0;
+  };
+  auto colsum = [&](const float* x, long long nrows, int C, float* out, float* out2) -> int {
+    const int L4 = (C < 256 ? C : 256) >> 2, lanes = 256 / L4;
+    long long blocks = (nrows + (long long)lanes * 8 - 1) / ((long long)lanes * 8);
+    blocks = blocks > 592 ? 592 : (blocks < 1 ? 1 : blocks);
+    colsum_kernel<<<dim3((unsigned)blocks, (C + 255) / 256), 256, 0, st>>>(x, out, out2, nullptr, nrows, C, C);
+    DMD_LAUNCH_OK();
+    return 0;
+  };
+  DMD_CUDA(cudaMemsetAsync(grads, 0, (size_t)core->grad_total * 4, st));
+  DMD_CUDA(cudaMemsetAsync(pl.zero_begin, 0, pl.zero_bytes, st));
+  // ---- head: logits = silu(y W0^T + b0) W2^T  (rew_end_model.py:35-39)
+  merge_logits_grad_kernel<<<(rows + 127) / 128, 128, 0, st>>>(g_logits_rew, g_logits_end, r.g_logits, b, t);
+  DMD_LAUNCH_OK();
+  if (sgemm(r.g_logits, 1, 5, r.hid, D, 1, G(h->i_h2w), D, 5, D, rows, 1)) return 1;                 // dW2 = g^T hid
+  if (sgemm(r.g_logits, 5, 1, W(h->i_h2w), D, 1, r.g_hid, D, rows, D, 5, 0)) return 1;               // g_hid = g W2
+  if (linear_launch(r.y, W(h->i_h0w), W(h->i_h0b), r.hpre, rows, D, D, 0, st)) return 1;             // pre-activation again
+  dsilu_mul_kernel<<<(unsigned)(((long long)rows * D + 255) / 256), 256, 0, st>>>(r.hpre, r.g_hid, r.g_pre, (long long)rows * D);
+  DMD_LAUNCH_OK();
+  if (sgemm(r.g_pre, 1, D, r.y, D, 1, G(h->i_h0w), D, D, D, rows, 1)) return 1;                      // dW0 = g_pre^T y
+  if (colsum(r.g_pre, rows, D, G(h->i_h0b), nullptr)) return 1;
+  if (sgemm(r.g_pre, D, 1, W(h->i_h0w), D, 1, r.g_y, D, rows, D, D, 0)) return 1;                    // g_y = g_pre W0
+  // ---- LSTM, backward through time: g_h(k) = g_y(k) + dgates(k+1) W_hh ; g_c carried in two ping-pong buffers
+  for (int k = t - 1, cur = 0; k >= 0; --k, cur ^= 1) {
+    float* gyk = r.g_y + (size_t)k * b * D;
+    if (k + 1 < t && sgemm(r.dgates + (size_t)(k + 1) * b * 4 * D, 4 * D, 1, W(h->i_whh), D, 1, gyk, D, b, D, 4 * D, 1)) return 1;
+    const float* cprev = k ? r.cells + (size_t)(k - 1) * b * D : r.zeros;
+    lstm_cell_bwd_kernel<<<(b * D + 255) / 256, 256, 0, st>>>(r.gates + (size_t)k * b * 4 * D, cprev, gyk, k + 1 < t ? r.g_c[cur] : nullptr,
+                                                             r.dgates + (size_t)k * b * 4 * D, r.g_c[cur ^ 1], b, D);
+    DMD_LAUNCH_OK();
+  }
+  // parameter gradients of all steps at once; x is the NCHW flatten of the encoder output (rew_end_model.py:52)
+  if (dmd_nhwc_to_nchw(pl.enc_out.data, r.x_flat, rows, h->feat_c, h->feat_c, h->feat_hw, st)) return 1;
+  if (sgemm(r.dgates, 1, 4 * D, r.x_flat, K, 1, G(h->i_wih), K, 4 * D, K, rows, 1)) return 1;                   // dW_ih = dgates^T x
+  if (t > 1 && sgemm(r.dgates + (size_t)b * 4 * D, 1, 4 * D, r.y, D, 1, G(h->i_whh), D, 4 * D, D, rows - b, 1)) return 1;   // dW_hh = sum_k dgates(k)^T h(k-1)
+  if (colsum(r.dgates, rows, 4 * D, G(h->i_bih), G(h->i_bhh))) return 1;
+  if (sgemm(r.dgates, 4 * D, 1, W(h->i_wih), K, 1, r.g_xflat, K, rows, K, 4 * D, 0)) return 1;                  // g_x = dgates W_ih
+  // ---- encoder: the feature gradient (NHWC) enters the fp16 tensor-core backward under a power-of-two loss scale
+  float* gfeat = pl.enc_out.grad;
+  if (dmd_nchw_to_nhwc(r.g_xflat, gfeat, rows, h->feat_c, h->feat_c, h->feat_hw, st)) return 1;
+  const long long n = (long long)rows * K;
+  absmax_kernel<<<(int)std::min<long long>((n + 255) / 256, 1184), 256, 0, st>>>(gfeat, pl.amax, n);
+  DMD_LAUNCH_OK();
+  loss_scale_kernel<<<1, 1, 0, st>>>(pl.amax, pl.scale);
+  DMD_LAUNCH_OK();
+  scale_inplace_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(gfeat, pl.scale, n);
+  DMD_LAUNCH_OK();
+  return run_bops(core, pl, grads, st);
 }

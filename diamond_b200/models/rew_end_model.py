@@ -4,17 +4,22 @@ The reward / termination model runs once per imagined step between the sampler a
 over the burn-in frames of every fresh episode (:120-129).  Parameters live under the reference's names (state_dict keys,
 `Agent.load`, `configure_opt`'s isinstance split keep working); the arithmetic — encoder ResBlocks at C = 32 with FiLM on
 the action embedding, two attention blocks, LSTM over time, SiLU head — runs in `dmd_rew_end_predict`.
-Training of this model (`forward`, rew_end_model.py:57-90) is the next row (f2) and is not built."""
+
+Training (`forward`, rew_end_model.py:57-90; SURVEY.md 8 f2) is native too: the host logic of the reference (final-frame
+substitution, mask, cross-entropy losses, confusion matrices) is torch on the device, and everything with FLOPs is one
+autograd node, `_RewEndFn`: `dmd_rew_end_forward_train` keeps the activations, `dmd_rew_end_backward` writes every parameter
+gradient into one flat buffer whose views become `.grad`."""
 import ctypes as C
 from dataclasses import dataclass
 from typing import List, Optional, Tuple
 
 import torch
 import torch.nn as nn
+import torch.nn.functional as F
 from torch import Tensor
 
 from .. import _lib
-from ..utils import NativeStateMixin, init_lstm
+from ..utils import LossAndLogs, NativeStateMixin, init_lstm
 from .blocks import Downsample, ResBlocks, _NativeOnly, conv3x3
 
 
@@ -132,5 +137,131 @@ class RewEndModel(NativeStateMixin, nn.Module):
                                            self._ws.numel(), _lib.current_stream()))
         return rew, end, (hx_o.unsqueeze(0), cx_o.unsqueeze(0))
 
-    def forward(self, batch):  # rew_end_model.py:57-90
-        raise NotImplementedError("RewEndModel training (SURVEY.md 8 f2) is not built; predict_rew_end (f1) is native")
+    # ------------------------------------------------------------------ training plumbing
+    def grad_layout(self):
+        """(offsets, numels, total) of the flat fp32 gradient buffer the native backward fills (state_dict order)."""
+        lib = _lib.lib()
+        h = self._native()
+        n = lib.dmd_rew_end_num_tensors(h)
+        offs, nums = (C.c_longlong * n)(), (C.c_longlong * n)()
+        total = lib.dmd_rew_end_grad_layout(h, offs, nums, n)
+        if total < 0:
+            raise RuntimeError("diamond_b200: " + lib.dmd_last_error().decode())
+        return list(offs), list(nums), int(total)
+
+    def acquire_train_workspace(self, nbytes: int) -> Tensor:
+        """A training workspace holds one forward's activations until its backward has run; pooled across steps."""
+        pool = self.__dict__.setdefault("_tws_pool", [])
+        for i, ws in enumerate(pool):
+            if ws.numel() >= nbytes and ws.device == self.device:
+                return pool.pop(i)
+        return torch.empty(nbytes, dtype=torch.uint8, device=self.device)
+
+    def release_train_workspace(self, ws: Tensor) -> None:
+        pool = self.__dict__.setdefault("_tws_pool", [])
+        if len(pool) < 2:
+            pool.append(ws)
+
+    def _check_frames(self, obs: Tensor) -> None:
+        s = self.cfg.img_size
+        if obs.dim() != 5 or obs.shape[-2:] != (s, s) or obs.shape[2] != self.cfg.img_channels:
+            raise RuntimeError(f"diamond_b200: rew_end frames must be (b, t, {self.cfg.img_channels}, {s}, {s}) (img_size of the "
+                               f"config), got {tuple(obs.shape)}")
+
+    # ------------------------------------------------------------------ reference surface
+    def forward(self, batch) -> LossAndLogs:  # rew_end_model.py:57-90
+        obs = batch.obs[:, :-1]
+        act = batch.act[:, :-1]
+        next_obs = batch.obs[:, 1:]
+        rew = batch.rew[:, :-1]
+        end = batch.end[:, :-1]
+        mask = batch.mask_padding[:, :-1]
+
+        # :67-71 when dead, the frame after the last step (padding) becomes the true final observation.  next_obs is a view:
+        # the assignment writes through into batch.obs, so the frame is also obs of the following step, as in the reference
+        dead = end.bool().any(dim=1)
+        if dead.any():
+            final_obs = torch.stack([i["final_observation"] for i, d in zip(batch.info, dead) if d]).to(obs.device)
+            next_obs[dead, end[dead].argmax(dim=1)] = final_obs
+
+        if torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
+            names = [k for k, _ in self.named_parameters()]
+            params = [p for _, p in self.named_parameters()]
+            logits_rew, logits_end = _RewEndFn.apply(self, names, obs, act, next_obs, *params)
+        else:
+            self._check_frames(obs)
+            logits_rew, logits_end, _ = self.predict_rew_end(obs, act, next_obs)
+        logits_rew = logits_rew[mask]
+        logits_end = logits_end[mask]
+        target_rew = rew[mask].sign().long().add(1)  # clipped to {-1, 0, 1}
+        target_end = end[mask]
+
+        loss_rew = F.cross_entropy(logits_rew, target_rew)
+        loss_end = F.cross_entropy(logits_end, target_end)
+        loss = loss_rew + loss_end
+
+        metrics = {
+            "loss_rew": loss_rew.detach(),
+            "loss_end": loss_end.detach(),
+            "loss_total": loss.detach(),
+            "confusion_matrix": {
+                "rew": confusion_matrix(logits_rew, target_rew, 3),
+                "end": confusion_matrix(logits_end, target_end, 2),
+            },
+        }
+        return loss, metrics
+
+
+def confusion_matrix(logits: Tensor, target: Tensor, num_classes: int) -> Tensor:
+    """torcheval's multiclass_confusion_matrix as the reference calls it (rew_end_model.py:84-85): int64 [n, n], rows the true
+    class, columns the arg-max prediction."""
+    n = num_classes
+    idx = target.long() * n + logits.detach().argmax(dim=1)
+    return torch.bincount(idx, minlength=n * n).reshape(n, n)
+
+
+class _RewEndFn(torch.autograd.Function):
+    """predict_rew_end from a zero LSTM state under autograd: forward = dmd_rew_end_forward_train (activations stay in the
+    training workspace), backward = dmd_rew_end_backward (all parameter gradients in one flat buffer, returned as views).
+    The frames and actions get no gradient."""
+
+    @staticmethod
+    def forward(ctx, module, names, obs, act, next_obs, *params):
+        lib = _lib.lib()
+        h = module._native()
+        module._check_frames(obs)
+        b, t = obs.shape[:2]
+        dev = obs.device
+        obs_, nxt_, act_ = obs.detach().float().contiguous(), next_obs.detach().float().contiguous(), act.long().contiguous()
+        rew = torch.empty(b, t, 3, device=dev)
+        end = torch.empty(b, t, 2, device=dev)
+        need = lib.dmd_rew_end_train_workspace_bytes(h, b, t)
+        if need == 0:
+            raise RuntimeError("diamond_b200: " + lib.dmd_last_error().decode())
+        ws = module.acquire_train_workspace(need)
+        _lib.check(lib.dmd_rew_end_forward_train(h, b, t, obs_.data_ptr(), nxt_.data_ptr(), act_.data_ptr(), rew.data_ptr(),
+                                                 end.data_ptr(), ws.data_ptr(), ws.numel(), _lib.current_stream()))
+        ctx.module, ctx.names, ctx.bt, ctx.ws, ctx.keep = module, names, (b, t), ws, (obs_, nxt_, act_)
+        return rew, end
+
+    @staticmethod
+    def backward(ctx, g_rew, g_end):
+        lib = _lib.lib()
+        module = ctx.module
+        h = module._native()
+        b, t = ctx.bt
+        dev = ctx.ws.device
+        g_rew = torch.zeros(b, t, 3, device=dev) if g_rew is None else g_rew.float().contiguous()
+        g_end = torch.zeros(b, t, 2, device=dev) if g_end is None else g_end.float().contiguous()
+        offs, nums, total = module.grad_layout()
+        flat = torch.empty(total, dtype=torch.float32, device=dev)
+        _lib.check(lib.dmd_rew_end_backward(h, b, t, g_rew.data_ptr(), g_end.data_ptr(), flat.data_ptr(), total, ctx.ws.data_ptr(),
+                                            _lib.current_stream()))
+        index = {k: i for i, k in enumerate(module.state_dict().keys())}
+        grads = []
+        for name, p in zip(ctx.names, module.parameters()):
+            i = index[name]
+            grads.append(flat[offs[i]:offs[i] + nums[i]].view_as(p))
+        module.release_train_workspace(ctx.ws)
+        module.last_flat_grad = flat   # one contiguous buffer: what a data-parallel step all-reduces in a single collective
+        return (None, None, None, None, None, *grads)

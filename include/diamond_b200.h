@@ -334,6 +334,22 @@ int dmd_rew_end_predict(dmd_rew_end* h, int b, int t, const float* obs, const fl
                         const float* hx_in, const float* cx_in, float* logits_rew, float* logits_end, float* hx_out,
                         float* cx_out, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- Reward / termination training: RewEndModel.forward under autograd (src/models/rew_end_model.py:57-90; trained in
+ * turn with the denoiser and the actor-critic, src/trainer.py:349-388).  dmd_rew_end_forward_train = predict_rew_end from a
+ * zero LSTM state that keeps every activation (encoder, the gates and cell states of all t LSTM steps, head input) in the
+ * training workspace, on a plan of its own: a later dmd_rew_end_predict is unaffected.  dmd_rew_end_backward consumes
+ * them: given dL/dlogits it writes (assigns) the gradient of EVERY parameter into one flat fp32 buffer (16-byte aligned
+ * slices in state_dict order, layout from dmd_rew_end_grad_layout).  The head and the LSTM backward run in fp32; the
+ * encoder backward on tcgen05 with a power-of-two loss scale chosen on the device from max|dL/dfeatures|. */
+size_t dmd_rew_end_train_workspace_bytes(dmd_rew_end* h, int b, int t);   /* 0 (dmd_last_error) when b, t are invalid */
+long long dmd_rew_end_grad_layout(const dmd_rew_end* h, long long* offsets, long long* numels, int n);
+/* obs / next_obs (b, t, C, S, S) fp32, act (b, t) int64 -> logits_rew (b, t, 3), logits_end (b, t, 2). */
+int dmd_rew_end_forward_train(dmd_rew_end* h, int b, int t, const float* obs, const float* next_obs, const int64_t* act,
+                              float* logits_rew, float* logits_end, void* workspace, size_t workspace_bytes, void* stream);
+/* g_logits_rew (b, t, 3), g_logits_end (b, t, 2); `workspace` is the forward's, untouched since. */
+int dmd_rew_end_backward(dmd_rew_end* h, int b, int t, const float* g_logits_rew, const float* g_logits_end, float* grads,
+                         long long grads_numel, void* workspace, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
